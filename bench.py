@@ -6,11 +6,13 @@
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
          bench.py --gpus N --steps K --warmup W               # one rank per GPU, batch-parallel
   ... bench.py --gpus N --workload PEMS07 --mode node         # node-sharded TSFormer + one NCCL all-gather
+  python bench.py --steps 10 --warmup 3 --dump-outputs DIR  # + the last timed step's outputs and gradients as .npy
 
 A "step" = one training step of STEP_<workload> (METR-LA: N=207 nodes, per-GPU batch 32, 168 patches of 12 = 2016-step
 long history): forward (frozen TSFormer in train() exactly as the reference runs it, discrete graph learning, Graph
 WaveNet), step_loss, backward to every trainable parameter (+ NCCL gradient all-reduce when N > 1).  Synthetic N(0,1)
-inputs, real pre-trained TSFormer weights for METR-LA (tests/golden fixture), seeded random GWNet/DGL weights.
+inputs, real pre-trained TSFormer weights for METR-LA (tests/golden fixture), seeded random GWNet/DGL weights; dropout
+and Gumbel seeds derive from a fixed torch seed, so the same arguments give the same inputs in every run.
 Prints ONE JSON line.
 """
 import argparse
@@ -24,6 +26,7 @@ import tempfile
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -31,6 +34,9 @@ sys.path.insert(0, ROOT)
 
 # (nodes, per-GPU batch, patches) of the reference's STEP_<NAME>.py configs (SURVEY section 8)
 WORKLOADS = {"METR-LA": (207, 32, 168), "PEMS04": (307, 8, 336), "PEMS-BAY": (325, 32, 168), "PEMS07": (883, 4, 168)}
+# --dump-outputs: the largest array (discrete_graph_learning.fc.weight's gradient, 38 M values at METR-LA) is sampled
+DUMP_MAX_ELEMS = 1 << 21
+DUMP_MAX_BYTES = 64 << 20
 
 
 def metric_name(ds):
@@ -69,7 +75,17 @@ def parse():
     ap.add_argument("--precision", default=os.environ.get("STEP_B200_PRECISION", "bf16"), choices=["bf16", "fp32"],
                     help="TSFormer encoder kernels: bf16 tcgen05 tensor cores (default, BASELINE config) or fp32 CUDA cores")
     ap.add_argument("--chunk-seqs", type=int, default=int(os.environ.get("STEP_B200_TS_CHUNK", "0")))
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (y_hat, theta, adj_knn, gsl_coefficient, "
+                         "loss and every trainable parameter's gradient) as DIR/<name>.npy in float32, so that two builds "
+                         "can be compared output for output; arrays over %d elements are written as a fixed sample"
+                         % DUMP_MAX_ELEMS)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
 
 
 # --------------------------------------------------------------------------------------------- helpers
@@ -150,27 +166,42 @@ def ts_state(ds):
     return torch.load(os.path.join(ROOT, "tests", "golden", "tsformer_METR-LA_state.pt"))
 
 
+def dump_sample(t):
+    """t itself, or, above DUMP_MAX_ELEMS elements, one element of every stride-wide window of the flattened tensor at
+    offsets drawn from a generator seeded by its size: every run and every build samples the same entries."""
+    t = t.detach()
+    n = t.numel()
+    if n <= DUMP_MAX_ELEMS:
+        return t
+    stride = n // DUMP_MAX_ELEMS
+    g = torch.Generator().manual_seed(n)
+    idx = torch.arange(DUMP_MAX_ELEMS) * stride + torch.randint(stride, (DUMP_MAX_ELEMS,), generator=g)
+    return t.reshape(-1)[idx.to(t.device)]
+
+
+def dump_outputs(arm, out_dir):
+    """Writes what the arm's last train_step handed its caller: the model's 4-tuple, the loss and the gradient of every
+    trainable parameter (the fp32 values an optimiser step would consume)."""
+    y_hat, theta, adj_knn, coeff, loss = arm.last_outputs
+    arrays = {"y_hat": y_hat, "theta": theta, "adj_knn": adj_knn, "gsl_coefficient": torch.tensor(coeff), "loss": loss}
+    for name, p in arm.model.named_parameters():
+        if p.grad is not None:
+            arrays["grad." + name] = p.grad
+    arrays = {k: dump_sample(v).to(torch.float32).cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes (limit %d)" % (total, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    sys.stderr.write("bench.py: %d arrays, %.1f MB written to %s\n" % (len(arrays), total / 1e6, out_dir))
+
+
 # --------------------------------------------------------------------------------------------- CPU comparator
-def _import_reference():
-    """The UNMODIFIED reference modules, importable only where /root/reference exists (the build container): the shims
-    are tests/golden/make_golden.py's (timm.trunc_normal_, empty easytorch, basicts.utils.load_pkl)."""
-    if not os.path.isdir("/root/reference/step/step_arch"):
-        return None
-    try:
-        import importlib.util
-        spec = importlib.util.spec_from_file_location("make_golden", os.path.join(ROOT, "tests", "golden", "make_golden.py"))
-        mg = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mg)
-        return mg.import_reference()
-    except Exception as e:          # noqa: BLE001  (any import problem -> fall back to the port, and say so)
-        sys.stderr.write("bench.py: reference import failed (%r); timing the oracle port instead\n" % (e,))
-        return None
-
-
 def cpu_reference_run(ds, steps, warmup, batch, dropout=True):
-    """The reference's CPU path on the host cores: the imported reference itself when /root/reference is present
-    (kind "reference"), else oracle/step_oracle.py's restatement (kind "port").  Same config except a bounded
-    per-step batch.  Returns (samples/s, info)."""
+    """The reference's CPU path on the host cores, run through oracle/step_oracle.py's restatement of its torch modules
+    (kind "port"; tests/test_oracle_golden.py holds the restatement to the reference's own outputs).  Same config except
+    a bounded per-step batch.  Returns (samples/s, info)."""
     from oracle import step_oracle as O
     nodes, _, patches = WORKLOADS[ds]
     # torch CPU ops on these shapes slow down badly past ~16-32 threads (measured on the 128-thread GPU host:
@@ -182,57 +213,21 @@ def cpu_reference_run(ds, steps, warmup, batch, dropout=True):
     sd.update({"tsformer." + k: v for k, v in ts_state(ds).items()})
     node_feats = O.synthetic_node_feats(ds, 0)
     history, long_history, future, uniform = O.synthetic_batch(ds, batch, patches, 0)
-    ref = None if os.environ.get("STEP_B200_CPU_KIND") == "port" else _import_reference()
     times = []
-    if ref is not None:
-        arch, dglmod, ref_loss = ref
-        tmp = tempfile.mkdtemp(prefix="step_ref_")
-        write_dataset(tmp, ds, node_feats)
-        torch.save({"model_state_dict": ts_state(ds)}, os.path.join(tmp, "ts.pt"))
-        cwd = os.getcwd()
-        os.chdir(tmp)
-        try:
-            model = arch.STEP(ds, os.path.join(tmp, "ts.pt"), ts_args(patches), gw_args(nodes),
-                              dict(dataset_name=ds, k=10, input_seq_len=12, output_seq_len=12))
-        finally:
-            os.chdir(cwd)
-        model.load_state_dict(sd, strict=True)
-        model.train()
-        if not dropout:
-            for m in model.modules():
-                if isinstance(m, torch.nn.Dropout):
-                    m.p = 0.0
-                if isinstance(m, torch.nn.MultiheadAttention):
-                    m.dropout = 0.0
-                if hasattr(m, "dropout") and isinstance(getattr(m, "dropout"), float):
-                    m.dropout = 0.0
-        for i in range(warmup + steps):
-            t0 = time.perf_counter()
-            y_hat, theta, adj_knn, coeff = model(history_data=history, long_history_data=long_history, future_data=None,
-                                                 batch_seen=0, epoch=1)
-            loss = ref_loss(y_hat[..., [0]], future[..., [0]], theta, adj_knn, coeff, null_val=0.0)
-            model.zero_grad(set_to_none=True)
-            loss.backward()
-            if i >= warmup:
-                times.append(time.perf_counter() - t0)
-        kind = "reference"
-    else:
+    for k in params:
+        sd[k] = sd[k].clone().requires_grad_(True)
+    for i in range(warmup + steps):
+        t0 = time.perf_counter()
+        loss, _ = O.train_step(sd, history, long_history, future, node_feats, uniform, epoch=1, null_val=0.0,
+                               gw_drop=0.3 if dropout else 0.0, ts_drop=0.1 if dropout else 0.0)
+        loss.backward()
         for k in params:
-            sd[k] = sd[k].clone().requires_grad_(True)
-        for i in range(warmup + steps):
-            t0 = time.perf_counter()
-            loss, _ = O.train_step(sd, history, long_history, future, node_feats, uniform, epoch=1, null_val=0.0,
-                                   gw_drop=0.3 if dropout else 0.0, ts_drop=0.1 if dropout else 0.0)
-            loss.backward()
-            for k in params:
-                sd[k].grad = None
-            if i >= warmup:
-                times.append(time.perf_counter() - t0)
-        kind = "port"
+            sd[k].grad = None
+        if i >= warmup:
+            times.append(time.perf_counter() - t0)
     dt = sum(times) / len(times)
-    what = ("the imported reference (step.step_arch.STEP + step_loss, unmodified)" if kind == "reference"
-            else "oracle/step_oracle.py (restatement of the reference's torch modules; /root/reference is not on this host)")
-    return batch / dt, {"cores": torch.get_num_threads(), "kind": kind,
+    what = "oracle/step_oracle.py (restatement of the reference's torch modules)"
+    return batch / dt, {"cores": torch.get_num_threads(), "kind": "port",
                         "sample": f"{steps} timed fwd+bwd steps (after {warmup} warm-up) of STEP_{ds} at batch {batch} "
                                   f"(CPU samples/s is ~flat in batch), fp32, dropout {'live as in the reference train()' if dropout else 'off'}, "
                                   f"{dt:.2f} s/step; {what}"}
@@ -351,6 +346,8 @@ class Arm:
         y_hat, theta, adj_knn, coeff = self.model(history_data=history, long_history_data=long_history, future_data=None,
                                                   batch_seen=0, epoch=1)
         loss = self.step_loss(y_hat[..., :1], future[..., :1], theta, adj_knn, coeff, null_val=0.0)
+        # detached: holding the graph would keep the backward's saved tensors alive into the next step
+        self.last_outputs = (y_hat.detach(), theta.detach(), adj_knn.detach(), coeff, loss.detach())
         self.reducer.zero()
         loss.backward()
         # NCCL all-reduce (big tensor in place + one packed buffer) when world > 1, enqueued on a side stream: it is joined
@@ -701,6 +698,8 @@ def main():
             arm.finish()
     ms_res = timed(resident_step, args.steps, dev, world)
     launches = int(_lib.load().step_launch_count()) - k0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(arm, args.dump_outputs)
     if args.only_resident:
         if rank == 0:
             sampler.stop()
