@@ -202,6 +202,24 @@ int step_tc_attention(const void *q_img, const void *k_img, const void *v_img, v
  * >= the threshold half (NaN patterns compare false): exactly floor(65536 p) of the 65536 patterns are dropped for
  * p >= 254/65536 (tests/test_host_logic.py enumerates them). */
 unsigned int step_tc_attn_drop_threshold(float drop_p);
+/* ---- stage-1 (pre-training) attention on tcgen05, bf16 operands / fp32 accumulation and statistics, P <= 352 ----
+ * Bytes of the log2-sum-exp buffer L [S, 4, P] fp32 the forward writes for the backward. */
+size_t step_tc_attn_train_lse_bytes(int S, int P);
+/* fp32 qkv rows [S*P, 288] (the in-projection output: q | k | v, head h at columns 24h..) -> the Q / K / V operand images
+ * of step_tc_qkv (sizes from step_tc_attn_image_bytes; Q pre-scaled by log2(e)/sqrt(24); every pad row written as zero).
+ * `bound` (may be NULL): the row-bound workspace step_tc_attention reads, filled as step_tc_qkv fills it. */
+int step_tc_attn_train_pack(const float *qkv, int S, int P, void *q_img, void *k_img, void *v_img, float *bound, void *stream);
+/* Training forward: out [S*P, 96] fp32 = dropout(softmax(q k^T / sqrt(24))) v per (sequence, head) and lse = the per-row
+ * log2-sum-exp of the log2-domain scores.  Attention-probability dropout from the counter hash keyed by `seed`
+ * (keep probability exactly 1 - floor(65536 p) / 65536, see step_tc_attn_train_keep_mask). */
+int step_tc_attn_train_fwd(const void *q_img, const void *k_img, const void *v_img, int S, int P, float drop_p,
+                           unsigned long long seed, float *out, float *lse, void *stream);
+/* Training backward: dqkv [S*P, 288] fp32 (every column of every row written) from the images, the forward's out and lse,
+ * and dout [S*P, 96]; the dropout mask is regenerated from (drop_p, seed). */
+int step_tc_attn_train_bwd(const void *q_img, const void *k_img, const void *v_img, const float *out, const float *lse,
+                           const float *dout, int S, int P, float drop_p, unsigned long long seed, float *dqkv, void *stream);
+/* Test helper: mask [S, 4, P, P] uint8 = 1 where the forward and backward above keep the probability (query row, key column). */
+int step_tc_attn_train_keep_mask(int S, int P, float drop_p, unsigned long long seed, unsigned char *mask, void *stream);
 size_t step_ts_encoder_bf16_workspace_bytes(int B, int N, int P);
 /* Whole encoder in bf16: series -> hidden [B,N,P,96] fp32 (same contract as step_ts_encoder_fwd). */
 int step_ts_encoder_fwd_bf16(const float *series, long long sB, long long sT, long long sN, int B, int N, int P,

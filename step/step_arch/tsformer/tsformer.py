@@ -147,6 +147,9 @@ class TSFormer(nn.Module):
         # "bf16": tcgen05 tensor-core kernels (bf16 operands, fp32 accumulation/statistics) - the performance path;
         # "fp32": CUDA-core kernels that meet the 1e-4 parity bar against the reference.
         self.precision = os.environ.get("STEP_B200_PRECISION", "bf16")
+        # stage-1 training (pretrain_forward_autograd) only: "bf16" runs the attention of every layer with P' <= 352 on
+        # tcgen05 (bf16 operands, fp32 accumulation/statistics); "fp32" keeps the CUDA-core attention kernels.
+        self.pretrain_precision = os.environ.get("STEP_B200_PRETRAIN_PRECISION", "fp32")
         self._tc_images = None
         self._tc_key = None
         self.seq_image = None        # bf16 Gram operand of the last bf16 forward ([B][P*12][R][8]); None in fp32 mode
@@ -253,11 +256,19 @@ class TSFormer(nn.Module):
         label_masked = label.reshape(B, N, -1).transpose(1, 2)
         return recon_masked, label_masked
 
+    def _pretrain_tc_attention(self, seq_len: int) -> bool:
+        """Whether stage-1 training runs the attention of a layer over `seq_len` tokens on the tensor cores: pretrain_precision
+        "bf16" and seq_len <= 352 (longer sequences keep the fp32 kernels, as in :meth:`encoding`)."""
+        if self.pretrain_precision not in ("bf16", "fp32"):
+            raise ValueError(f"TSFormer.pretrain_precision must be 'bf16' or 'fp32', got {self.pretrain_precision!r}")
+        return self.pretrain_precision == "bf16" and seq_len <= 352
+
     def pretrain_forward_autograd(self, history_data):
         """The same ``mode="pre-train"`` computation as :meth:`pretrain_forward`, built from differentiable ops (every one
         a hand-written kernel behind ``step_b200.ops``: split-bf16 tcgen05 GEMMs for the dense layers, fp32 attention /
-        LayerNorm / dropout kernels with hand-written backward) so that stage 1 of STEP - the masked auto-encoder of
-        reference tsformer.py:71-160 - trains on the GPU.  Gradients reach all 72 parameters."""
+        LayerNorm / dropout kernels with hand-written backward; with ``pretrain_precision="bf16"`` the attention runs on
+        tcgen05 instead) so that stage 1 of STEP - the masked auto-encoder of reference tsformer.py:71-160 - trains on
+        the GPU.  Gradients reach all 72 parameters."""
         B, N, _, T = history_data.shape
         L, d = self.patch_size, self.embed_dim
         P = T // L
@@ -270,13 +281,14 @@ class TSFormer(nn.Module):
         ui = torch.as_tensor(unmasked, device=dev, dtype=torch.long)
         mi = torch.as_tensor(masked, device=dev, dtype=torch.long)
         nu, nm = len(unmasked), len(masked)
+        tc_attn = self._pretrain_tc_attention
         # --- patch + positional embedding (dropout on every token, positional_encoding.py:32), keep the unmasked 25 %
         patches = history_data[:, :, self.selected_feature, :].reshape(S * P, L)
         tok = ops.Linear.apply(patches, emb.weight.view(d, L), emb.bias, False).view(S, P, d) + pos[:P]
         tok = ops.dropout(tok.reshape(S * P, d), drop, seed, 1).view(S, P, d)
         z = (tok.index_select(1, ui) * math.sqrt(d)).reshape(S * nu, d)
         for i, lw in enumerate(self.encoder.kernel_weights()):
-            z = ops.transformer_layer_train(z, S, nu, lw, drop, seed, 16 * (i + 1))
+            z = ops.transformer_layer_train(z, S, nu, lw, drop, seed, 16 * (i + 1), tc_attention=tc_attn(nu))
         z = ops.AddLayerNorm.apply(z, None, self.encoder_norm.weight, self.encoder_norm.bias)
         # --- decoder over [unmasked | mask tokens + positional embedding of the masked positions]
         dec_u = ops.Linear.apply(z, self.enc_2_dec_emb.weight, self.enc_2_dec_emb.bias, False).view(S, nu, d)
@@ -284,7 +296,7 @@ class TSFormer(nn.Module):
         dec_m = ops.dropout(dec_m.reshape(S * nm, d), drop, seed, 2).view(S, nm, d)
         z = (torch.cat([dec_u, dec_m], dim=1) * math.sqrt(d)).reshape(S * P, d)
         for i, lw in enumerate(self.decoder.kernel_weights()):
-            z = ops.transformer_layer_train(z, S, P, lw, drop, seed, 160 + 16 * i)
+            z = ops.transformer_layer_train(z, S, P, lw, drop, seed, 160 + 16 * i, tc_attention=tc_attn(P))
         z = ops.AddLayerNorm.apply(z, None, self.decoder_norm.weight, self.decoder_norm.bias)
         recon = ops.Linear.apply(z, self.output_layer.weight, self.output_layer.bias, False).view(B, N, P, L)
         recon_masked = recon[:, :, nu:, :].reshape(B, N, -1).transpose(1, 2)

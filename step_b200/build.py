@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libstep_b200.so")
-SOURCES = ["ts_encoder.cu", "ts_train.cu", "tc_encoder.cu", "graph_learn.cu", "trunk.cu", "trunk_fc.cu", "tc_gemm.cu", "gw_glue.cu", "optim.cu", "gwnet.cu"]
+SOURCES = ["ts_encoder.cu", "ts_train.cu", "tc_encoder.cu", "tc_attn_train.cu", "graph_learn.cu", "trunk.cu", "trunk_fc.cu", "tc_gemm.cu", "gw_glue.cu", "optim.cu", "gwnet.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
 

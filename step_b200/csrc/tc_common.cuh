@@ -256,4 +256,42 @@ __device__ __forceinline__ void unpack8_bf16(uint4 u, float *v) {
   }
 }
 
+__device__ __forceinline__ float fast_exp2(float x) {
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+
+// ---- counter hash of the tensor-core dropout sites (lowbias32-style finaliser: 2 multiplies + 2 xor-shifts) -------------
+__device__ __forceinline__ uint32_t hash32(uint32_t x) {
+  x *= 0x9E3779B1u; x ^= x >> 16; x *= 0x85EBCA77u; x ^= x >> 15;
+  return x;
+}
+
+// ---- attention-probability dropout: two keep decisions per 32-bit random word -------------------------------------
+// Each half of the word is compared AS A bf16 NUMBER with a threshold (one HSET2.BF16 for two elements, result 0xFFFF /
+// 0x0000 per half, applied to the packed bf16 probabilities with one AND).  As numbers the 65536 patterns order as
+// -inf = 0xFF80 < ... < 0x8001 < -0 = +0 < 0x0001 < ... < +inf, and the 254 NaN patterns fail every comparison, so
+// "dropped" = NaNs + the (D - 254) most negative patterns for D = p * 65536 dropped patterns out of 65536: the keep
+// probability is exactly 1 - D / 65536 for p >= 254 / 65536 (smaller p are served as 254 / 65536).
+__host__ __device__ inline uint32_t drop_thr_bf16x2(uint32_t thr16) {
+  const uint32_t need = thr16 > 254u ? thr16 - 254u : 0u;
+  uint32_t t;
+  if (need <= 32640u) t = 0xFF80u - need;
+  else { t = need - 32641u; if (t > 0x7F80u) t = 0x7F80u; }
+  return t | (t << 16);
+}
+__device__ __forceinline__ uint32_t keep_mask_bf16x2(uint32_t r, uint32_t thr2) {
+  uint32_t m;
+  asm("set.ge.u32.bf16x2 %0, %1, %2;" : "=r"(m) : "r"(r), "r"(thr2));
+  return m;
+}
+
+// Placement of a (head, row tile) of the attention Q image in the 128 TMEM lanes: a last tile of <= 64 queries sits at
+// lanes 64.. for odd heads, so that the partial tiles of consecutive heads are exponentiated by warps of different SM
+// sub-partitions.
+__host__ __device__ __forceinline__ int q_tail_offset(int P, int rt, int h) {
+  return ((P - rt * 128) <= 64 && (h & 1)) ? 64 : 0;
+}
+
 }  // namespace tc

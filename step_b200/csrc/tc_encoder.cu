@@ -22,15 +22,11 @@ constexpr int HD = 24;                           // head dim
 
 enum { TCM_F32 = 0, TCM_RELU_IMG = 1, TCM_RESLN = 2, TCM_QKV = 3 };
 
-// Dropout masks of the tensor-core path: one counter hash (lowbias32-style finaliser: 2 multiplies + 2 xor-shifts)
-// seeds each group of 8 consecutive elements, a 32-bit LCG step per element (one IMAD) walks the group, and the full
-// 32-bit state is compared with the threshold (keep probability exactly 1 - thr16 / 65536).  ~4 integer ops per
-// element instead of ~50 for Philox4x32-10, which matters because TSFormer draws 3.0 G attention-probability masks
-// per step; still counter-based, so a mask is a pure function of (seed, site, element index).
-__device__ __forceinline__ uint32_t hash32(uint32_t x) {
-  x *= 0x9E3779B1u; x ^= x >> 16; x *= 0x85EBCA77u; x ^= x >> 15;
-  return x;
-}
+// Dropout masks of the tensor-core path: one counter hash (hash32 in tc_common.cuh) seeds each group of 8 consecutive
+// elements, a 32-bit LCG step per element (one IMAD) walks the group, and the full 32-bit state is compared with the
+// threshold (keep probability exactly 1 - thr16 / 65536).  ~4 integer ops per element instead of ~50 for
+// Philox4x32-10, which matters because TSFormer draws 3.0 G attention-probability masks per step; still counter-based,
+// so a mask is a pure function of (seed, site, element index).
 __device__ __forceinline__ void drop8(float *v, uint64_t idx8, uint32_t thr16, float scale, uint64_t key) {
   const uint32_t salt = (uint32_t)key ^ ((uint32_t)(key >> 32) * 0x9E3779B9u) ^ ((uint32_t)(idx8 >> 32) * 0x85EBCA6Bu);
   uint32_t st = hash32((uint32_t)idx8 ^ salt);
@@ -40,35 +36,6 @@ __device__ __forceinline__ void drop8(float *v, uint64_t idx8, uint32_t thr16, f
     st = st * 2891336453u + 1013904223u;          // full-period LCG mod 2^32 (L'Ecuyer multiplier); high bits decide
     v[i] = (st >= thr) ? v[i] * scale : 0.f;
   }
-}
-__device__ __forceinline__ float fast_exp2(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-
-// ---- attention-probability dropout: two keep decisions per 32-bit random word -------------------------------------
-// Each half of the word is compared AS A bf16 NUMBER with a threshold (one HSET2.BF16 for two elements, result 0xFFFF /
-// 0x0000 per half, applied to the packed bf16 probabilities with one AND).  As numbers the 65536 patterns order as
-// -inf = 0xFF80 < ... < 0x8001 < -0 = +0 < 0x0001 < ... < +inf, and the 254 NaN patterns fail every comparison, so
-// "dropped" = NaNs + the (D - 254) most negative patterns for D = p * 65536 dropped patterns out of 65536: the keep
-// probability is exactly 1 - D / 65536 for p >= 254 / 65536 (smaller p are served as 254 / 65536).
-__host__ __device__ inline uint32_t drop_thr_bf16x2(uint32_t thr16) {
-  const uint32_t need = thr16 > 254u ? thr16 - 254u : 0u;
-  uint32_t t;
-  if (need <= 32640u) t = 0xFF80u - need;
-  else { t = need - 32641u; if (t > 0x7F80u) t = 0x7F80u; }
-  return t | (t << 16);
-}
-__device__ __forceinline__ uint32_t keep_mask_bf16x2(uint32_t r, uint32_t thr2) {
-  uint32_t m;
-  asm("set.ge.u32.bf16x2 %0, %1, %2;" : "=r"(m) : "r"(r), "r"(thr2));
-  return m;
-}
-// Placement of a (head, row tile) in the 128 TMEM lanes: a last tile of <= 64 queries sits at lanes 64.. for odd heads, so
-// that the partial tiles of consecutive heads are exponentiated by warps of different SM sub-partitions.
-__host__ __device__ __forceinline__ int q_tail_offset(int P, int rt, int h) {
-  return ((P - rt * 128) <= 64 && (h & 1)) ? 64 : 0;
 }
 // One block of NC score columns of a row: p = 2^(s - m) (0 for columns >= `valid`), row sums, dropout, bf16 K-major image.
 // `dst` points at this row's 16-byte slot of the block's first 8-column chunk; chunks at or beyond `chunks` are not stored.

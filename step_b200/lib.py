@@ -69,6 +69,11 @@ SIGNATURES = {
     "step_tc_attn_drop_threshold": (C.c_uint, [C.c_float]),
     "step_tc_qkv": (C.c_int, [vp, vp, f32p, C.c_int, C.c_int, vp, vp, vp, f32p, vp]),
     "step_tc_attention": (C.c_int, [vp, vp, vp, vp, f32p, C.c_int, C.c_int, C.c_float, ull, vp]),
+    "step_tc_attn_train_lse_bytes": (C.c_size_t, [C.c_int, C.c_int]),
+    "step_tc_attn_train_pack": (C.c_int, [f32p, C.c_int, C.c_int, vp, vp, vp, f32p, vp]),
+    "step_tc_attn_train_fwd": (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_float, ull, f32p, f32p, vp]),
+    "step_tc_attn_train_bwd": (C.c_int, [vp, vp, vp, f32p, f32p, f32p, C.c_int, C.c_int, C.c_float, ull, f32p, vp]),
+    "step_tc_attn_train_keep_mask": (C.c_int, [C.c_int, C.c_int, C.c_float, ull, vp, vp]),
     "step_ts_encoder_bf16_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "step_ts_encoder_fwd_bf16": (C.c_int, [f32p, ll, ll, ll, C.c_int, C.c_int, C.c_int, f32p, f32p, f32p,
                                            C.POINTER(TsLayerWeights), C.POINTER(TsLayerImages), C.c_int, f32p, f32p, f32p, vp, vp,

@@ -171,6 +171,69 @@ class Attention(torch.autograd.Function):
         return dqkv, None, None, None, None
 
 
+ATTN_TC_MAX_P = 352     # longest sequence the tensor-core attention holds (K and V of one head stay in shared memory)
+
+
+def attention_tc_pack(qkv: Tensor, S: int, P: int, bound: bool = False):
+    """fp32 qkv rows [S*P, 288] -> (q_img, k_img, v_img[, bound]) bf16 operand images of the tensor-core attention."""
+    qkv = _f32(qkv, "qkv")
+    st = _enter(qkv)
+    L = _L()
+    q_img = torch.empty(L.step_tc_attn_image_bytes(S, P, 0), device=qkv.device, dtype=torch.uint8)
+    k_img = torch.empty(L.step_tc_attn_image_bytes(S, P, 1), device=qkv.device, dtype=torch.uint8)
+    v_img = torch.empty_like(k_img)
+    bnd = torch.empty(L.step_tc_attn_image_bytes(S, P, 2) // 4, device=qkv.device, dtype=torch.float32) if bound else None
+    check(L.step_tc_attn_train_pack(qkv.data_ptr(), S, P, q_img.data_ptr(), k_img.data_ptr(), v_img.data_ptr(), _p(bnd), st),
+          "step_tc_attn_train_pack")
+    launch_counter["kernels"] += 1
+    return (q_img, k_img, v_img, bnd) if bound else (q_img, k_img, v_img)
+
+
+def attention_tc_keep_mask(S: int, P: int, drop_p: float, seed: int, device) -> Tensor:
+    """[S, 4, P, P] uint8, 1 where AttentionTC keeps the attention probability (query row, key column) - for tests."""
+    mask = torch.empty(S, 4, P, P, device=device, dtype=torch.uint8)
+    st = _enter(mask)
+    check(_L().step_tc_attn_train_keep_mask(S, P, float(drop_p), int(seed) & (2**64 - 1), mask.data_ptr(), st),
+          "step_tc_attn_train_keep_mask")
+    return mask
+
+
+class AttentionTC(torch.autograd.Function):
+    """Same contract as :class:`Attention` (qkv [S*P, 288] -> [S*P, 96]) on tcgen05: bf16 Q/K/V operands, fp32 accumulation
+    and softmax statistics, P <= 352.  Keeps the operand images, O and the per-row log2-sum-exp for the backward, which
+    recomputes the probabilities on the tensor cores.  Attention-probability dropout uses the tensor-core counter hash
+    (not :class:`Attention`'s Philox stream: same distribution, different masks)."""
+
+    @staticmethod
+    def forward(ctx, qkv, S, P, drop_p, seed):
+        S, P = int(S), int(P)
+        if P > ATTN_TC_MAX_P:
+            raise _lib.StepB200Error(f"AttentionTC: P={P} > {ATTN_TC_MAX_P}; use Attention")
+        q_img, k_img, v_img = attention_tc_pack(qkv, S, P)
+        out = torch.empty(S * P, 96, device=qkv.device, dtype=torch.float32)
+        lse = torch.empty(S * 4 * P, device=qkv.device, dtype=torch.float32)
+        seed = int(seed) & (2**64 - 1)
+        st = _enter(qkv)
+        check(_L().step_tc_attn_train_fwd(q_img.data_ptr(), k_img.data_ptr(), v_img.data_ptr(), S, P, float(drop_p), seed,
+                                          out.data_ptr(), lse.data_ptr(), st), "step_tc_attn_train_fwd")
+        launch_counter["kernels"] += 1
+        ctx.save_for_backward(q_img, k_img, v_img, out, lse)
+        ctx.cfg = (S, P, float(drop_p), seed)
+        return out
+
+    @staticmethod
+    def backward(ctx, dout):
+        q_img, k_img, v_img, out, lse = ctx.saved_tensors
+        S, P, drop_p, seed = ctx.cfg
+        dout = _f32(dout, "dout")
+        st = _enter(dout)
+        dqkv = torch.empty(S * P, 288, device=dout.device, dtype=torch.float32)
+        check(_L().step_tc_attn_train_bwd(q_img.data_ptr(), k_img.data_ptr(), v_img.data_ptr(), out.data_ptr(), lse.data_ptr(),
+                                          dout.data_ptr(), S, P, drop_p, seed, dqkv.data_ptr(), st), "step_tc_attn_train_bwd")
+        launch_counter["kernels"] += 1
+        return dqkv, None, None, None, None
+
+
 class AddLayerNorm(torch.autograd.Function):
     """LayerNorm96(x + r) (r may be None): the post-norm residual blocks and the final norms of the transformer."""
 
@@ -226,11 +289,14 @@ def dropout(x: Tensor, p: float, seed: int, site: int) -> Tensor:
     return Dropout.apply(x, p, seed, site) if p > 0.0 else x
 
 
-def transformer_layer_train(z: Tensor, S: int, P: int, lw: Dict[str, Tensor], drop_p: float, seed: int, site: int) -> Tensor:
+def transformer_layer_train(z: Tensor, S: int, P: int, lw: Dict[str, Tensor], drop_p: float, seed: int, site: int,
+                            tc_attention: bool = False) -> Tensor:
     """One post-norm nn.TransformerEncoderLayer(96, 4, 384) on tokens z [S*P, 96] with autograd (stage-1 training path;
-    the forecasting path uses the fused inference kernels)."""
+    the forecasting path uses the fused inference kernels).  tc_attention: attention on tcgen05 (:class:`AttentionTC`,
+    P <= 352) instead of the fp32 kernels."""
     qkv = Linear.apply(z, lw["in_proj_w"], lw["in_proj_b"], False)
-    o = Attention.apply(qkv, S, P, drop_p, (seed + 7919 * site) & (2**63 - 1))
+    attn = AttentionTC if tc_attention else Attention
+    o = attn.apply(qkv, S, P, drop_p, (seed + 7919 * site) & (2**63 - 1))
     o = dropout(Linear.apply(o, lw["out_proj_w"], lw["out_proj_b"], False), drop_p, seed, site + 2)
     z1 = AddLayerNorm.apply(z, o, lw["norm1_w"], lw["norm1_b"])
     f = dropout(Linear.apply(z1, lw["lin1_w"], lw["lin1_b"], True), drop_p, seed, site + 3)
